@@ -227,7 +227,13 @@ def main():
     ap.add_argument('--no-extra', action='store_true', help='skip the C2 / C5 sub-results of the default line')
     ap.add_argument('--graph', type=int, default=int(os.environ.get('HD_GRAPH', '1')),
                     help='1 = replay the device-resident step from a CUDA graph (one graph launch per step), 0 = eager launches')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write the outputs of the last timed step as DIR/<name>.npy (float32, at most 64 MB in '
+                         'all: larger arrays are cut to a fixed seeded sample along their longest axis); inputs are seeded, so runs '
+                         'with the same arguments can be compared output for output')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.warmup < 3 and args.impl == 'ours':
         args.warmup = 3
 
@@ -378,6 +384,11 @@ def main():
     if args.workload != 'smpl':
         sel_idx = [0, B - 1]
         timed_out = {k: last['out'][k][sel_idx].float().cpu().numpy() for k in PARITY_KEYS if k in last['out']}
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # what a caller of the timed path receives: the fetch keys (not the '_'-prefixed inspection buffers) / the SMPL outputs
+        res = outs if args.workload == 'smpl' else last['out']
+        dumped = dump_outputs({k: v for k, v in res.items() if not k.startswith('_') and v is not None}, args.dump_outputs)
     gather_ok = None
     if world > 1 and rank == 0 and last.get('g') is not None:
         # gathered tensors must contain rank 0's own clips bit for bit (the N-GPU == 1-GPU identity is tests/test_multi_gpu.py);
@@ -515,6 +526,8 @@ def main():
             line['cpu_baseline'] = cpu_baseline
         if extra:
             line['extra'] = extra
+        if dumped is not None:
+            line['dumped_outputs'] = {'dir': args.dump_outputs, 'shapes': dumped}
         if parity:
             line['parity'] = parity
             if 'parity_max_rel' in parity:
@@ -529,6 +542,33 @@ def main():
     if world > 1:
         dist.destroy_process_group()
     return 0
+
+
+DUMP_BYTES = 60 << 20       # --dump-outputs: array data in all; with the .npy headers the files stay under 64 MB (64e6 bytes)
+
+
+def dump_outputs(outs, path, budget=DUMP_BYTES):
+    """Writes each output tensor as path/<name>.npy in float32.  Smaller arrays are written whole; the budget left over is shared
+    among the larger ones, each cut down, while over its share, along its longest axis to a sorted sample of indices drawn with a
+    fixed seed.  The sample depends only on the shapes, so two builds run with the same arguments write comparable files."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    items = sorted(outs.items(), key=lambda kv: (kv[1].numel(), kv[0]))
+    left, written = budget, {}
+    for i, (name, t) in enumerate(items):
+        share = left // (len(items) - i)
+        t = t.detach()
+        rng = np.random.RandomState(0)
+        while t.numel() * 4 > share:
+            ax = max(range(t.dim()), key=lambda d: t.shape[d])
+            keep = max(1, t.shape[ax] * share // (t.numel() * 4))
+            idx = np.sort(rng.choice(t.shape[ax], keep, replace=False))
+            t = t.index_select(ax, torch.from_numpy(idx).to(t.device))
+        a = t.float().cpu().numpy()
+        np.save(os.path.join(path, name + '.npy'), a)
+        left -= a.nbytes
+        written[name] = list(a.shape)
+    return written
 
 
 def workload_name(args):

@@ -17,8 +17,12 @@ unpinned" still means for this repo; see oracle/ref_exec/README.md.
 Inputs are not stored: they are regenerated from seeds by human_dynamics_b200.synthetic (weights seed 1, SMPL seed 2, ...),
 exactly as listed in CASES below; large outputs are stored sub-sampled (130 vertices).
 
-Only runs where /root/reference exists (this container).  Run from the repo root:
-    python tests/golden/make_ref_exec_golden.py            (about 2 minutes, ~3 GB RAM, writes ~0.5 GB to a temp dir)
+Needs a checkout of the reference, named by HD_REFERENCE_ROOT.  Run from the repo root:
+    HD_REFERENCE_ROOT=<reference checkout> python tests/golden/make_ref_exec_golden.py          (about 2 minutes, ~3 GB RAM,
+                                                                                               writes ~0.5 GB to a temp dir)
+    HD_REFERENCE_ROOT=<reference checkout> python tests/golden/make_ref_exec_golden.py sweeps   (ref_sweeps_v1.npz)
+    HD_REFERENCE_ROOT=<reference checkout> python tests/golden/make_ref_exec_golden.py regen    (ref_exec_regen_v1.npz: the cheap
+                                                                                               sections again, in a run of their own)
 """
 import importlib.util
 import os
@@ -31,7 +35,7 @@ import types
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-REF = os.environ.get('HD_REFERENCE_ROOT', '/root/reference')
+REF = os.environ.get('HD_REFERENCE_ROOT', '')
 STUBS = os.path.join(ROOT, 'oracle', 'ref_exec', 'stubs')
 VERT_IDS = np.arange(0, 6890, 53)
 
@@ -46,8 +50,8 @@ def _by_path(name, path):
 def setup_paths():
     """`src` must resolve to the REFERENCE package (this repo has a drop-in package of the same name), `tensorflow` etc. to
     the stand-ins.  Repo helpers (synthetic inputs, checkpoint writer) are loaded by file path, never through sys.path."""
-    if not os.path.isdir(os.path.join(REF, 'src')):
-        raise SystemExit('reference tree not found at %s' % REF)
+    if not REF or not os.path.isdir(os.path.join(REF, 'src')):
+        raise SystemExit('set HD_REFERENCE_ROOT to a checkout of the reference (got %r)' % REF)
     for p in (ROOT, os.path.join(ROOT, 'tests'), ''):
         while p in sys.path:
             sys.path.remove(p)
@@ -146,16 +150,19 @@ def gen_models(out, syn, weights):
     assign_all()
     out['resnet64_phi'] = sess.run(phi)
     out['resnet_var_names'] = np.array(sorted(v.op_name for v in tf.global_variables()))
-    # az_fc2_groupnorm (models.py:121-228)
+    # az_fc2_groupnorm (models.py:121-228); 2048-wide outputs are stored at every 16th channel + checksums of all channels
+    sc = _by_path('_sweep_cases', os.path.join(ROOT, 'tests', 'golden', 'sweep_cases.py'))
     rng = np.random.RandomState(42)
     x = rng.normal(0, 1, size=(2, 20, 2048)).astype(np.float32)
     y = models.az_fc2_groupnorm(is_training=False, net=tf.constant(x), num_conv_layers=3)
     assign_all()
-    out['fmovie_out'] = sess.run(y)
+    y = sess.run(y)
+    out['fmovie_out'], out['fmovie_out_proj'] = y[..., ::16], sc.checksum(y, lead=2)
     # fc2_res (models.py:270-296)
     z = models.fc2_res(tf.constant(x))
     assign_all()
-    out['fc2res_out'] = sess.run(z)
+    z = sess.run(z)
+    out['fc2res_out'], out['fc2res_out_proj'] = z[..., ::16], sc.checksum(z, lead=2)
     # batch_pred_omega -> call_hmr_ief -> hmr_ief -> encoder_fc3_dropout (models.py:233-267,299-415,80-116)
     B, T = 2, 5
     feats = rng.normal(0, 1, size=(B, T, 2048)).astype(np.float32)
@@ -325,8 +332,102 @@ def gen_eval_util(out):
     out['ev_rot2aa'] = np.asarray(E.rot_mat_to_axis_angle(Rm))
 
 
+def gen_sweeps(out, syn, tmp):
+    """Wider sweeps than the fixture above, stored in ref_sweeps_v1.npz; their inputs come from sweep_cases.py."""
+    import cv2
+    import tensorflow as tf
+    from src import models
+    from src.evaluation import eval_util as E
+    from src.evaluation.run_video import process_image
+    from src.evaluation.tester import Tester
+    from src.tf_smpl.batch_smpl import SMPL
+    from src.tf_smpl.projection import batch_orth_proj_idrot
+    sc = _by_path('_sweep_cases', os.path.join(ROOT, 'tests', 'golden', 'sweep_cases.py'))
+    # eval_util.py metrics; per-case results of equal shape are stacked along a first axis of cases
+    cases = {}
+    for i, (gt, pr, vis, kg, kp) in enumerate(sc.eval_sweep()):
+        e, pa = E.compute_error_3d(gt, pr)
+        ek, epa, pck = E.compute_error_kp(kg, kp)
+        for key, a in (('e', e), ('pa', pa), ('sim', E.compute_similarity_transform(pr[0], gt[0])), ('ek', ek), ('epa', epa), ('pck', pck),
+                       ('verts', E.compute_error_verts(gt, pr))):
+            cases.setdefault('ev_' + key, []).append(np.asarray(a, np.float64))
+        out['ev_acc_%d' % i] = np.asarray(E.compute_error_accel(gt, pr, vis))       # length = number of visible frame triples
+    out.update((k, np.stack(v)) for k, v in cases.items())
+    # tester.py:260-312 sliding window, `predict` replaced by a probe returning the frame ids it was shown
+    for ci, (N, B, T, L) in enumerate(sc.SLIDING_CASES):
+        t = Tester.__new__(Tester)
+        t.batch_size, t.sequence_length, t.img_size, t.fov = B, T, 2, L * 4 + 1
+        t.predict = lambda images: {'ids': np.asarray(images)[:, :, 0, 0, 0].copy(), 'two': np.asarray(images)[:, :, :, 0, 0] * 2.0}
+        r = t.predict_all_images(sc.sliding_frames(N, np.float64))
+        out['sw_ids_%d' % ci], out['sw_two_%d' % ci] = np.asarray(r['ids']), np.asarray(r['two'])
+    # models.py with 2 temporal blocks, B=3, T=7, delta heads (-3, +3)
+    tf.reset_default_graph()
+    w, x, om0 = sc.other_config_inputs(syn)
+    y = models.get_temporal_encoder()(is_training=False, net=tf.constant(x), num_conv_layers=2)
+    om, deltas = models.batch_pred_omega(input_features=y, batch_size=3, is_training=False, num_output=85, omega_mean=tf.constant(om0),
+                                         sequence_length=7, scope='single_view_ief', predict_delta_keys=[3, 0, -3],
+                                         use_delta_from_pred=True, use_optcam=True)
+    for v in tf.global_variables():
+        v.load(w[v.op_name])
+    r = tf.Session().run({'strips': y, 'omega': om, 'dm3': deltas[-3], 'dp3': deltas[3]})
+    out['mo_strips'], out['mo_strips_proj'] = r['strips'][..., ::16], sc.checksum(r['strips'], lead=2)
+    out['mo_omega'], out['mo_dm3'], out['mo_dp3'] = r['omega'], r['dm3'], r['dp3']
+    out['mo_names'] = np.array(sorted(v.op_name for v in tf.global_variables()))
+    tf.reset_default_graph()
+    # SMPL / batch_lbs with large rotations and the dense-weight 19-keypoint model
+    pkl = os.path.join(tmp, 'smpl_dense.pkl')
+    write_smpl_pickle(sc.smpl_sweep_model(syn), pkl)
+    beta, theta, cam = sc.smpl_sweep_inputs()
+    s = SMPL(pkl)
+    v, j, R = s(tf.constant(beta), tf.constant(theta), get_skin=True)
+    k = batch_orth_proj_idrot(j, tf.constant(cam))
+    r = tf.Session().run({'verts': v, 'joints': j, 'Rs': R, 'Jtr': s.J_transformed, 'kps': k})
+    out['sm_verts'], out['sm_verts_proj'] = r['verts'][:, sc.VERT_IDS], sc.checksum(r['verts'])
+    out['sm_joints'], out['sm_Rs'], out['sm_Jtr'], out['sm_kps'] = r['joints'], r['Rs'], r['Jtr'], r['kps']
+    tf.reset_default_graph()
+    # run_video.py:56-107 process_image, frames handed over as (lossless) PNG files through its imread; one row per case
+    cases = {}
+    for i, (H, W, cx, cy, s, frame) in enumerate(sc.process_image_sweep()):
+        path = os.path.join(tmp, 'sweep_%d.png' % i)
+        cv2.imwrite(path, cv2.cvtColor(frame, cv2.COLOR_RGB2BGR))
+        r = process_image(path, np.array([cx, cy, s], np.float64))
+        img = np.asarray(r['image'], np.float64)
+        for key, a in (('frame_sum', frame.astype(np.int64).sum()), ('shape', img.shape),
+                       ('meta', list(r['center']) + list(r['start_pt']) + list(r['im_shape']))):
+            cases.setdefault('pi_' + key, []).append(np.asarray(a, np.int64))
+        cases.setdefault('pi_sample', []).append(sc.pixel_sample(img, i))
+        cases.setdefault('pi_proj', []).append(sc.checksum(img[None])[0])
+    out.update((k, np.stack(v)) for k, v in cases.items())
+
+
 def main():
     syn, ckpt = setup_paths()
+    if sys.argv[1:2] == ['regen']:
+        # the fixture's cheap sections (SMPL path, process_image, eval metrics) regenerated in a run of their own
+        tmp = tempfile.mkdtemp(prefix='ref_regen_')
+        out = {}
+        try:
+            write_smpl_pickle(syn.make_synthetic_smpl(seed=2), os.path.join(tmp, 'smpl.pkl'))
+            gen_smpl(out, syn, os.path.join(tmp, 'smpl.pkl'))
+            gen_process_image(out, tmp)
+            gen_eval_util(out)
+        finally:
+            shutil.rmtree(tmp, ignore_errors=True)
+        path = sys.argv[2] if len(sys.argv) > 2 else os.path.join(ROOT, 'tests', 'golden', 'ref_exec_regen_v1.npz')
+        np.savez_compressed(path, **out)
+        print('wrote', path, os.path.getsize(path), 'bytes,', len(out), 'arrays')
+        return
+    if sys.argv[1:] == ['sweeps']:
+        tmp = tempfile.mkdtemp(prefix='ref_sweeps_')
+        out = {}
+        try:
+            gen_sweeps(out, syn, tmp)
+        finally:
+            shutil.rmtree(tmp, ignore_errors=True)
+        path = os.path.join(ROOT, 'tests', 'golden', 'ref_sweeps_v1.npz')
+        np.savez_compressed(path, **out)
+        print('wrote', path, os.path.getsize(path), 'bytes,', len(out), 'arrays')
+        return
     weights = syn.make_synthetic_weights(seed=1, with_hal=True)
     smpl = syn.make_synthetic_smpl(seed=2)
     tmp = tempfile.mkdtemp(prefix='ref_exec_')
